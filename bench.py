@@ -132,6 +132,34 @@ class ClockSampler:
                 "source": "NVML, 10 ms period, timed region only"}
 
 
+DUMP_BYTES = 60_000_000
+
+
+def dump_outputs(dirname: str, b, sol: np.ndarray, info: np.ndarray):
+    """What the timed path returned in its last step, as float64 .npy files under DUMP_BYTES in all: the per-QP info fields
+    and input trajectories of every QP, and the whole solution records of a fixed, seeded sample of QPs (sorted rows in
+    sol_rows.npy).  When even the per-QP arrays of every QP do not fit, they are taken on one seeded sample of rows too
+    (qp_rows.npy), of which the solution records are a subset."""
+    os.makedirs(dirname, exist_ok=True)
+    nb = b.nbatch
+    out = {f: info[f].astype(np.float64) for f in ("status", "iter", "res_max", "mu", "obj", "dual_gap", "lq_count")}
+    out["u"] = b.layout.u_traj(sol)
+    rng = np.random.default_rng(0)
+    row_bytes = sum(a.nbytes for a in out.values()) // nb + 8
+    if row_bytes * nb > DUMP_BYTES // 2:
+        qp_rows = np.sort(rng.choice(nb, DUMP_BYTES // 2 // row_bytes, replace=False))
+        out = {name: a[qp_rows] for name, a in out.items()}
+        out["qp_rows"] = qp_rows.astype(np.float64)
+    else:
+        qp_rows = np.arange(nb)
+    room = DUMP_BYTES - sum(a.nbytes for a in out.values())
+    k = min(len(qp_rows), room // (8 * (b.layout.sol_stride + 1)))
+    rows = np.sort(rng.choice(qp_rows, k, replace=False))
+    out["sol_rows"], out["sol"] = rows.astype(np.float64), np.ascontiguousarray(sol[rows])
+    for name, a in out.items():
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
 def cpu_reference(batch_obj, opts, nqp: int, threads: int = 0):
     """Times the unmodified reference on the host cores on the first nqp QPs of the workload."""
     from acados_b200.problems import Batch
@@ -180,7 +208,11 @@ def main():
     ap.add_argument("--no-plugin", action="store_true", help="skip the end-to-end leg through the plugin's batched entry")
     ap.add_argument("--no-tight", action="store_true", help="skip the second parity pass (all tolerances 1e-12)")
     ap.add_argument("--config", default="c2", choices=sorted(CONFIGS), help="BASELINE.json configuration (default c2: the one the metric is quoted on)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="", help="write what the timed path returned in its last step to DIR/<name>.npy "
+                    "(float64, at most 60 MB; rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     global _CONFIG, METRIC
     _CONFIG = args.config
     if args.batch <= 0:
@@ -205,15 +237,17 @@ def main():
             return 0
         sample = args.cpu_sample or args.batch
         b = workload(sample, seed=1234)
-        times = []
-        base = None
+        solve_s, wall_s = [], []
         for it in range(warmup + steps):
-            t0 = time.perf_counter()
-            base, _, info = cpu_reference(b, opts, sample)
+            base, rsol, info = cpu_reference(b, opts, sample)
             if it >= warmup:
-                times.append(time.perf_counter() - t0)
-        # cpu_reference runs a 64-QP warm-up + the sample; use its own wall clock of the sample
-        val = base["value"]
+                # cpu_reference runs a 64-QP warm-up + the sample; use its own clocks of the sample
+                solve_s.append(sample / base["value"])
+                wall_s.append(sample / base["value_incl_struct_packing"])
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, b, rsol, info)
+        val = sample * steps / sum(solve_s)
+        base["value"], base["value_incl_struct_packing"] = val, sample * steps / sum(wall_s)
         line = {"metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": steps, "warmup": warmup,
                 "ms_per_step": 1e3 * sample / val, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
                 "dtype": "f64", "data": "synthetic", "impl": "reference", "config": config,
@@ -275,6 +309,8 @@ def main():
     launches_per_step = solver.last_launch_count
     clocks = sampler.stop()
     dev_ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, b, d_sol.cpu().numpy(), np.frombuffer(d_info.cpu().numpy().tobytes(), dtype=INFO_DTYPE))
     # per-launch duration of the solve kernel (events recorded around each launch by the solver itself)
     solver.solve_device(nb, d_qp.data_ptr(), d_sol.data_ptr(), d_info.data_ptr(), opts, sync=True)
     solve_ms = solver.last_kernel_ms                 # all kernels of one solve (repack, throughput kernel, generic kernel over hand-backs)

@@ -1,8 +1,9 @@
 """Solution sensitivities (reference: d_ocp_qp_ipm_sens_frw / _adj behind the plugin's eval_forw_sens / eval_adj_sens,
 external/hpipm/ocp_qp/x_ocp_qp_ipm.c:3285-3444): one substitution with the factorisation of the last IPM iteration.
 
-CPU part: the oracle's restatement against the unmodified reference.  GPU part: the CUDA path (cuipm_sens_host, through
-the C ABI) against the oracle.
+CPU part: the oracle's restatement against the unmodified reference, through its outputs stored by
+tests/golden/make_reference_outputs.py (a seeded sample of each sensitivity field with an entry in every stage, and the
+field's max |.|).  GPU part: the CUDA path (cuipm_sens_host, through the C ABI) against the oracle.
 
 Tolerances.  The sensitivities are evaluated at the last IPM iterate, where the slacks t of active constraints are
 1e-9..1e-16: an absolute difference of 1e-12 between two solvers' iterates (what the solve parity test allows) is a
@@ -11,11 +12,13 @@ with it.  So: instances on which the two SOLUTIONS agree to round-off (lam and t
 majority) must agree in dux / dpi / dt to 1e-9 relative, the others to 1e-2.  dlam (and the adjoint
 dt = dt / t) of active constraints are lam/t * (a difference of O(1) numbers that cancels to ~1e-11): the reference's own
 value carries ~1e-3 relative error there, those arrays are held to 2e-2 throughout."""
+import os
+
 import numpy as np
 import pytest
 
 from acados_b200.binding import default_opts
-from test_oracle_vs_reference import CASES
+from test_oracle_vs_reference import CASES, GOLD, input_fingerprint, ref_decode, reference_outputs
 
 SENS_CASES = ["c1_mass_spring", "c2_chain_mass", "rand_box", "rand_general", "rand_soft", "rand_masked", "rand_x0_free", "unconstrained"]
 
@@ -33,6 +36,7 @@ def _seed(b, which):
 
 
 def _check(b, e1, e2, adjoint, ok, s1, s2):
+    """e2: a sensitivity record, or a function (q, fld) -> max |a1 - a2| / max |a2| over field fld of QP q."""
     L = b.layout
     lt1 = np.concatenate([L.gather(s1, "lam"), L.gather(s1, "t")], axis=1)
     lt2 = np.concatenate([L.gather(s2, "lam"), L.gather(s2, "t")], axis=1)
@@ -42,10 +46,13 @@ def _check(b, e1, e2, adjoint, ok, s1, s2):
         tight = 1e-9 if agree[q] <= 1e-13 else 1e-2
         ntight += agree[q] <= 1e-13
         for fld in ("ux", "pi", "lam", "t"):
-            a1, a2 = L.gather(e1[q:q + 1], fld)[0], L.gather(e2[q:q + 1], fld)[0]
-            if a2.size == 0:
+            if callable(e2):
+                err = e2(q, fld)
+            else:
+                a1, a2 = L.gather(e1[q:q + 1], fld)[0], L.gather(e2[q:q + 1], fld)[0]
+                err = np.max(np.abs(a1 - a2)) / max(np.max(np.abs(a2)), 1e-300) if a2.size else None
+            if err is None:
                 continue
-            err = np.max(np.abs(a1 - a2)) / max(np.max(np.abs(a2)), 1e-300)
             loose = fld == "lam" or (fld == "t" and adjoint)
             assert err <= (2e-2 if loose else tight), (q, fld, err, agree[q])
     return ntight
@@ -55,16 +62,27 @@ def _check(b, e1, e2, adjoint, ok, s1, s2):
 @pytest.mark.parametrize("adjoint", [False, True])
 @pytest.mark.parametrize("which", ["ux", "lam", "all"])
 def test_oracle_sens_matches_reference(built, name, adjoint, which):
+    """The reference's solution is the golden one of tests/golden/<name>.npz (same solve); its sensitivities are compared on
+    the stored sample of every field, relative to the field's max |.| as in the full comparison."""
     from oracle import oracle_binding as ob
-    if not ob.have_ref():
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
     b = CASES[name]()
     seed = _seed(b, which)
     o = default_opts()
     s1, i1, e1 = ob.oracle_solve_sens(b, o, seed, adjoint=adjoint)
-    s2, i2, e2 = ob.ref_solve_sens(b, o, seed, adjoint=adjoint)
-    assert np.array_equal(i1["iter"], i2["iter"])
-    _check(b, e1, e2, adjoint, i2["status"] == 0, s1, s2)
+    z, key = reference_outputs("sens"), f"{name}/adj{int(adjoint)}/{which}"
+    assert np.allclose(input_fingerprint(b.qp), z[name + "/inputs"], rtol=1e-12, atol=0), "generator drifted from the stored inputs"
+    g = np.load(os.path.join(GOLD, name + ".npz"), allow_pickle=False)
+    assert np.array_equal(i1["iter"], z[key + "/iter"])
+
+    def err(q, fld):
+        if key + f"/{fld}/idx" not in z:
+            return None
+        v2, eps = ref_decode(z, key + f"/{fld}/val")
+        norm = z[key + f"/{fld}/norm"][q]
+        a1 = b.layout.gather(e1[q:q + 1], fld)[0, z[key + f"/{fld}/idx"]]
+        return np.max(np.abs(a1 / norm - v2[q])) + eps
+
+    _check(b, e1, err, adjoint, g["status"] == 0, s1, g["sol"])
 
 
 def test_sens_is_linear_in_the_seed(built):
